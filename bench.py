@@ -2,6 +2,7 @@
 """Headline benchmark: samples/s for full T=1000 DDPM sampling (999 UNet evaluations + posterior updates per sample).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4|cfg1|cfg5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Headline workload = BASELINE.json configs[2] (cfg3): the conditional Family-R UNet of ddpm_DANRA_conditional_wValid__128x128
@@ -20,6 +21,11 @@ configurations ride along as `secondary` objects (fewer steps; cfg2 64x64 batch 
 `--impl reference`: that same reference CPU implementation as its own arm — identical `config`, each step = one call of the
                reference's own DiffusionUtils.sample bounded to a few reverse steps of a sub-batch (`cpu_baseline.sample` says
                which); `ms_per_step` is the time actually measured, `value` the extrapolation to 999 steps per sample.
+`--dump-outputs DIR`: after the timed steps, the fields x_0 that the last timed step of the headline workload returned (the whole
+               global batch) go to DIR/x0.npy as float32 [B, C, H, W].  Inputs, weights and noise seeds depend only on the
+               arguments, so two builds run with the same arguments can be compared field for field.  Compare with a
+               tolerance: atomic reductions make two runs of one build differ in the last bits (cfg3, 256 fields on one B200
+               at its 1000 W limit: 7e-6 relative L2).
 """
 from __future__ import annotations
 
@@ -54,6 +60,7 @@ REF_SAMPLE = {"cfg1": (4, 8), "cfg2": (8, 4), "cfg3": (4, 2), "cfg4": (4, 2), "c
 HEAD_DIM_OF_CLASS = {"attn_tc": 16, "attn_tc32": 32}
 SFU_PEAK_TEXP = 4.63     # measured on this pool's B200s: tools/ub/mufu.cu (ex2.approx.ftz.f32, all SMs)
 NCU_TRAFFIC = {}         # filled from profiles/r2_ncu_traffic.json when present (dram bytes per launch, per kernel class)
+DUMP_BYTES = 64 << 20    # --dump-outputs writes at most this much
 
 
 def peaks():
@@ -62,6 +69,18 @@ def peaks():
         d = json.load(open(p))
         return dict(hbm=d["hbm_gbs"], tf_burst=d["bf16_tflops"], tf_sustained=d["bf16_tflops_sustained"], src="measured")
     return dict(hbm=6650.0, tf_burst=1590.0, tf_sustained=1400.0, src="fallback (B200_PROFILING.md)")
+
+
+def dump_outputs(path, x0):
+    """x0 as <path>/x0.npy (float32).  A batch above DUMP_BYTES is cut to a fixed sample of whole fields (seeded by 0, kept in
+    batch order), the same for every run with the same arguments."""
+    import numpy as np
+    x0 = x0.float().cpu()
+    if x0.numel() * 4 > DUMP_BYTES:
+        keep = torch.randperm(x0.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_BYTES // (x0[0].numel() * 4)]
+        x0 = x0[keep.sort().values]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "x0.npy"), x0.numpy())
 
 
 def workload_config(name, world):
@@ -221,8 +240,9 @@ class Bench:
             ms, wall = float(t[0].item()), float(t[1].item()) / 1e3
         return ms, wall, out
 
-    def run_workload(self, name, steps, warmup, e2e_steps, clocks=None, profile=False):
-        """Device-resident and host end-to-end throughput of one workload; returns a dict (rank 0 fills the roofline)."""
+    def run_workload(self, name, steps, warmup, e2e_steps, clocks=None, profile=False, keep_output=False):
+        """Device-resident and host end-to-end throughput of one workload; returns a dict (rank 0 fills the roofline).
+        keep_output: res["output"] holds the global batch of x_0 of the last timed device step, on the host."""
         import torch.distributed as dist
         from diffusionmodelscustom_b200 import DiffusionUtils
         from diffusionmodelscustom_b200.configs import build_ours_d, build_ours_r, inputs_d, inputs_r
@@ -270,6 +290,8 @@ class Bench:
                        "d2h_bytes_per_step": pinned["x"].numel() * 4 * world},
                "gpu_launches": int(launches), "fp16_saturations": net.saturation_count(),
                "tflops_per_gpu": value * WORKLOADS[name]["flops"] * (T_STEPS - 1) / 1e12 / world}
+        if keep_output:     # still the last timed device step: the host path writes neither x0 nor the gather buffers
+            res["output"] = (torch.cat(gather) if world > 1 else x0).cpu()
         if profile and rank == 0:
             tt = torch.full((batch,), 500, dtype=torch.long)
             res["profile"] = net.profile_step(d["x"], tt, d["y"], d["cond"], d["lsm"], d["topo"], reps=5)
@@ -361,7 +383,13 @@ def main():
                     "cfg5 = the 1024-member ensemble through the generation driver")
     ap.add_argument("--e2e-steps", type=int, default=0, help="timed host end-to-end steps (default min(steps, 3))")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write x_0 of the last timed step of the headline workload to DIR/x0.npy (float32, <= 64 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.global_batch:
         WORKLOADS[args.workload]["global_batch"] = args.global_batch
     rank = int(os.environ.get("RANK", "0"))
@@ -383,8 +411,11 @@ def main():
     B = Bench(rank, world, dev)
     sampler = ClockSampler(local_rank) if rank == 0 else None
     e2e_steps = args.e2e_steps or max(1, min(args.steps, 3))
-    head = B.run_workload(args.workload, args.steps, args.warmup, e2e_steps, sampler, profile=True)
+    head = B.run_workload(args.workload, args.steps, args.warmup, e2e_steps, sampler, profile=True,
+                          keep_output=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop() if sampler else None
+    if "output" in head:
+        dump_outputs(args.dump_outputs, head.pop("output"))
     secondary = {}
     for name in [s for s in args.secondary.split(",") if s and s != args.workload]:
         if name == "cfg5":
