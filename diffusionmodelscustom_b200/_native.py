@@ -18,7 +18,8 @@ INTERP_MODES = {"bicubic": 0, "bilinear": 1, "nearest": 2}
 SYMBOLS = ["b2d_last_error", "b2d_abi_version", "b2d_create", "b2d_destroy", "b2d_load_weights", "b2d_set_schedule",
            "b2d_set_conditioning", "b2d_forward", "b2d_sample", "b2d_sample_host", "b2d_last_launch_count", "b2d_debug_read", "b2d_profile_step",
            "b2d_op_conv2d", "b2d_op_layernorm", "b2d_op_attention", "b2d_op_attn_block", "b2d_op_attn_block_out", "b2d_op_instnorm", "b2d_op_posterior_update", "b2d_saturation_count", "b2d_debug_attn_trace", "b2d_ensemble_run",
-           "b2d_op_noise_image", "b2d_op_weighted_mse", "b2d_op_eval_daily", "b2d_op_eval_pixel", "b2d_op_histogram", "b2d_encoder_forward", "b2d_decoder_forward", "b2d_op_final_layer"]
+           "b2d_op_noise_image", "b2d_op_weighted_mse", "b2d_op_eval_daily", "b2d_op_eval_pixel", "b2d_op_histogram", "b2d_encoder_forward", "b2d_decoder_forward", "b2d_op_final_layer",
+           "b2d_set_timesteps", "b2d_op_ddim_update"]
 
 
 class Config(C.Structure):
@@ -79,6 +80,9 @@ def lib():
         L.b2d_op_final_layer.argtypes = [C.c_void_p] * 4 + [C.c_int32] * 4 + [C.c_void_p]
         L.b2d_op_posterior_update.argtypes = [C.c_void_p] * 6 + [C.c_int32, C.c_int32, C.c_int64, C.c_uint64, C.c_uint64,
                                                                  C.c_float, C.c_void_p]
+        L.b2d_set_timesteps.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_float]
+        L.b2d_op_ddim_update.argtypes = [C.c_void_p] * 4 + [C.c_int32] * 3 + [C.c_float, C.c_int32, C.c_int64, C.c_uint64,
+                                                              C.c_uint64, C.c_float, C.c_void_p]
         L.b2d_op_noise_image.argtypes = [C.c_void_p] * 6 + [C.c_int32, C.c_int64, C.c_uint64, C.c_uint64, C.c_float, C.c_void_p]
         L.b2d_op_weighted_mse.argtypes = [C.c_void_p] * 3 + [C.c_float, C.c_float, C.c_void_p, C.c_int64, C.c_void_p]
         L.b2d_op_eval_daily.argtypes = [C.c_void_p] * 4 + [C.c_int32, C.c_int64, C.c_void_p]

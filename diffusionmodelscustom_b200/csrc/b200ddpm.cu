@@ -112,6 +112,19 @@ struct Handle {
     // step for the remainder of (T-1) / graph_steps.
     cudaGraphExec_t graph_multi = nullptr, graph_one = nullptr;
     int graph_steps = 0, graph_nodes_multi = 0, graph_nodes_one = 0;
+    // DDIM sampler (b2d_set_timesteps): the sequence tau, its per-step coefficients and the step index k are device-resident, so
+    // its own graph pair depends on (program, schedule tables, has_y) like the DDPM pair and not on S; the two pairs coexist.
+    bool ddim = false;                 // sampler mode of sample_core: false = the reference DDPM loop
+    std::vector<int> ddim_tau;         // tau_0 > ... > tau_{S-1}
+    float ddim_eta = 0.f;
+    bool ddim_dirty = true;            // sequence, eta or schedule changed since the tables were uploaded
+    int ddim_cap = 0;                  // entries of d_ddim_tau (T + 1: S <= T-1 plus two trailing zeros)
+    int* d_ddim_tau = nullptr;
+    float4* d_ddim_coef = nullptr;     // [S] {cx, ce, sigma, 0} from ddim_coefficients()
+    int* d_t_next = nullptr;           // [max_batch] tau_{k+1}: the timestep the DDIM side branch embeds
+    cudaGraphExec_t graph_multi_ddim = nullptr, graph_one_ddim = nullptr;
+    int graph_nodes_multi_ddim = 0, graph_nodes_one_ddim = 0;
+    std::vector<float> h_alpha_hat;    // host copy of the schedule's alpha_hat (the DDIM coefficients are computed from it)
     SampleJob* d_job = nullptr;
     float* d_x_work = nullptr;       // [max_batch][c_hr][H][H] fp32: the diffusion state of the running job
     // host-entry staging (allocated once with the handle: no cudaMalloc/cudaFree inside b2d_sample_host)
@@ -128,7 +141,8 @@ struct Handle {
     int dec_begin_op = -1;
     struct Fmap { f16* p; int C, hw; } fmaps[5] = {};
     int temb_free_op = -1;   // index of the first step op after the last reader of d_temb (set by the program builders)
-    int temb_t_off = 0;      // added to d_t by the next temb launch (-1 on the side branch)
+    int* temb_t = nullptr;   // timesteps the next temb launch reads: d_t, or d_t_next on the DDIM side branch
+    int temb_t_off = 0;      // added to *temb_t by the next temb launch (-1 on the DDPM side branch)
     cudaStream_t side_stream = nullptr;
     cudaEvent_t ev_side_fork = nullptr, ev_side_join = nullptr;
     cudaEvent_t ev_br_fork = nullptr, ev_br_join = nullptr;   // Op::side / Op::join branches
@@ -150,10 +164,16 @@ struct Handle {
         taps.clear();
         prog_B = 0;
     }
+    void drop_ddim_graphs() {
+        if (graph_multi_ddim) cudaGraphExecDestroy(graph_multi_ddim);
+        if (graph_one_ddim) cudaGraphExecDestroy(graph_one_ddim);
+        graph_multi_ddim = graph_one_ddim = nullptr;
+    }
     void drop_graphs() {
         if (graph_multi) cudaGraphExecDestroy(graph_multi);
         if (graph_one) cudaGraphExecDestroy(graph_one);
         graph_multi = graph_one = nullptr;
+        drop_ddim_graphs();
     }
     // cudaFree of one long-lived allocation (schedule tables / noise staging that are re-sized)
     void release(void* p) {
@@ -700,7 +720,7 @@ static int build_program_r(Handle* h, int B) {
         ops.meta("temb", "temb_project", 2.0 * B * TS * 256, 4.0 * TS * 256);
         ops.push_back([=](cudaStream_t st) {
             dim3 grid((TS + TEMB_OC - 1) / TEMB_OC, (B + TEMB_SB - 1) / TEMB_SB);
-            B2D_CUDA(launch_k(temb_project_kernel, dim3(grid), dim3(256), 0, st, hh->d_t, hh->has_y ? hh->d_y : nullptr, label, ei, dd, tw, tb, temb, 1024,
+            B2D_CUDA(launch_k(temb_project_kernel, dim3(grid), dim3(256), 0, st, hh->temb_t, hh->has_y ? hh->d_y : nullptr, label, ei, dd, tw, tb, temb, 1024,
                                                       TS, B, hh->temb_t_off, hh->cfg.stem_embedding));
             B2D_CUDA(cudaGetLastError());
             return 0;
@@ -877,6 +897,7 @@ static int init_uniform_carveout() {
     B2D_TRY(set_carveout(instnorm_apply_kernel));
     B2D_TRY(set_carveout(tail_conv_kernel));
     B2D_TRY(set_carveout(posterior_update_kernel));
+    B2D_TRY(set_carveout(ddim_update_kernel));
     B2D_TRY(set_carveout(fill_int_kernel));
     B2D_TRY(set_carveout(bicubic_resize_kernel));
     B2D_TRY(set_carveout(linear_nearest_resize_kernel));
@@ -898,6 +919,8 @@ static int init_batch_buffers(Handle* h) {
     const b2d_config& c = h->cfg;
     const int B = c.max_batch, H = c.img_size;
     B2D_TRY(h->alloc(&h->d_t, B));
+    B2D_TRY(h->alloc(&h->d_t_next, B));
+    h->temb_t = h->d_t;
     B2D_TRY(h->alloc(&h->d_y, B));
     B2D_TRY(h->alloc(&h->d_step, 4));   // [0] step index i, [1] arrival counter of the posterior update (self-resetting)
     B2D_CUDA(cudaMemset(h->d_step, 0, 16));
@@ -928,8 +951,10 @@ static int ensure_program(Handle* h, int B) {
 
 // pipelined = inside the reverse loop: op 0 (time embeddings) of this step was produced by the previous step's side branch
 // (or by the loop prologue), and the embeddings of the NEXT step are launched on the side stream at temb_free_op.  The
-// caller joins the side branch (join_temb_side) before it advances the step counter.
-static int run_step_ops(Handle* h, cudaStream_t st, bool pipelined = false, int first = 0, int last = -1) {
+// caller joins the side branch (join_temb_side) before it advances the step counter.  The side branch runs before the update
+// that advances t, so it cannot read the next t from d_t: the DDPM loop embeds d_t - 1, the DDIM loop (ddim = true) embeds
+// d_t_next, which holds tau_{k+1} (a stride of more than one step).
+static int run_step_ops(Handle* h, cudaStream_t st, bool pipelined = false, int first = 0, int last = -1, bool ddim = false) {
     static const bool dbg = getenv("B2D_DEBUG_SYNC") != nullptr;
     static const bool no_pipe = getenv("B2D_NO_TEMB_PIPE") != nullptr;
     static const bool no_branch = getenv("B2D_NO_BRANCH") != nullptr;
@@ -963,8 +988,10 @@ static int run_step_ops(Handle* h, cudaStream_t st, bool pipelined = false, int 
         if (pipe && idx == h->temb_free_op) {
             B2D_CUDA(cudaEventRecord(h->ev_side_fork, st));
             B2D_CUDA(cudaStreamWaitEvent(h->side_stream, h->ev_side_fork, 0));
-            h->temb_t_off = -1;
+            if (ddim) h->temb_t = h->d_t_next;
+            else h->temb_t_off = -1;
             const int rc = h->step_ops[0](h->side_stream);
+            h->temb_t = h->d_t;
             h->temb_t_off = 0;
             if (rc) return rc;
             B2D_CUDA(cudaEventRecord(h->ev_side_join, h->side_stream));
@@ -986,6 +1013,36 @@ static bool temb_pipelined(const Handle* h) {
 }
 static int join_temb_side(Handle* h, cudaStream_t st) {
     if (temb_pipelined(h)) B2D_CUDA(cudaStreamWaitEvent(st, h->ev_side_join, 0));
+    return 0;
+}
+
+// Device tables of the DDIM loop for the current (schedule, sequence, eta): re-validated against T, re-computed and uploaded only
+// when one of them changed (this synchronises the device: queued work may still read the old tables).
+static int ddim_prepare(Handle* h) {
+    const int T = h->T, S = (int)h->ddim_tau.size();
+    B2D_CHECK(S >= 1 && h->ddim_tau[0] <= T - 1, "DDIM timesteps exceed T-1 of the current schedule");
+    B2D_CHECK((int)h->h_alpha_hat.size() == T, "internal: host alpha_hat out of date");
+    if (!h->ddim_dirty && h->ddim_cap >= T + 1) return 0;
+    B2D_CUDA(cudaDeviceSynchronize());
+    if (h->ddim_cap < T + 1) {
+        h->drop_ddim_graphs();   // they hold the table pointers
+        h->release(h->d_ddim_tau);
+        h->release(h->d_ddim_coef);
+        h->d_ddim_tau = nullptr;
+        h->d_ddim_coef = nullptr;
+        h->ddim_cap = 0;
+        B2D_TRY(h->alloc(&h->d_ddim_tau, T + 1));
+        B2D_TRY(h->alloc(&h->d_ddim_coef, T + 1));
+        h->ddim_cap = T + 1;
+    }
+    std::vector<int> tau(h->ddim_tau);
+    tau.resize(S + 2, 0);
+    std::vector<float4> coef(S);
+    for (int k = 0; k < S; ++k)
+        coef[k] = ddim_coefficients(h->h_alpha_hat[tau[k]], k + 1 < S ? h->h_alpha_hat[tau[k + 1]] : 1.0f, h->ddim_eta);
+    B2D_CUDA(cudaMemcpy(h->d_ddim_tau, tau.data(), tau.size() * sizeof(int), cudaMemcpyHostToDevice));
+    B2D_CUDA(cudaMemcpy(h->d_ddim_coef, coef.data(), coef.size() * sizeof(float4), cudaMemcpyHostToDevice));
+    h->ddim_dirty = false;
     return 0;
 }
 
@@ -1103,8 +1160,35 @@ int b2d_set_schedule(b2d_handle* h, const float* betas, const float* alphas, con
     B2D_CUDA(cudaMemcpy(h->d_betas, betas, T * 4, cudaMemcpyHostToDevice));
     B2D_CUDA(cudaMemcpy(h->d_alphas, alphas, T * 4, cudaMemcpyHostToDevice));
     B2D_CUDA(cudaMemcpy(h->d_alpha_hat, alpha_hat, T * 4, cudaMemcpyHostToDevice));
+    h->h_alpha_hat.assign(alpha_hat, alpha_hat + T);
+    h->ddim_dirty = true;
     return 0;
 }
+
+int b2d_set_timesteps(b2d_handle* h, const int32_t* timesteps_host, int32_t n, float eta) {
+    B2D_CHECK(h, "null handle");
+    if (n == 0) {
+        B2D_CHECK(timesteps_host == nullptr, "n == 0 restores the DDPM loop and takes no timesteps");
+        h->ddim = false;
+        return 0;
+    }
+    B2D_CHECK(timesteps_host && n >= 1, "timesteps: NULL or negative length");
+    B2D_CHECK(eta >= 0.f && eta <= 1.f, "eta must lie in [0, 1]");
+    for (int k = 0; k < n; ++k) {
+        B2D_CHECK(timesteps_host[k] >= 1, "timesteps must be >= 1");
+        B2D_CHECK(k == 0 || timesteps_host[k] < timesteps_host[k - 1], "timesteps must be strictly decreasing");
+    }
+    B2D_CHECK(h->T < 2 || timesteps_host[0] <= h->T - 1, "timesteps must be <= T-1 of the current schedule");
+    std::vector<int> tau(timesteps_host, timesteps_host + n);
+    if (tau != h->ddim_tau || eta != h->ddim_eta) {
+        h->ddim_tau.swap(tau);
+        h->ddim_eta = eta;
+        h->ddim_dirty = true;
+    }
+    h->ddim = true;
+    return 0;
+}
+
 
 // y_dev: int64 labels in device memory (synchronises once to range-check them, as nn.Embedding would raise);
 // y_host: the same in host memory (no device round trip).  At most one of them is non-null.
@@ -1254,26 +1338,31 @@ int b2d_decoder_forward(b2d_handle* h, const float* const* fmaps_in, const int64
     return 0;
 }
 
-// One reverse step on stream `st`: the eps program on d_x_work, then the posterior update (whose last block advances i and t).
-static int enqueue_reverse_step(b2d_handle* h, int B, cudaStream_t st) {
+// One reverse step on stream `st`: the eps program on d_x_work, then the posterior update (whose last block advances i and t),
+// or in DDIM mode the DDIM update (whose last block advances k, t and t_next).
+static int enqueue_reverse_step(b2d_handle* h, int B, cudaStream_t st, bool ddim) {
     const b2d_config& c = h->cfg;
     const size_t per_sample = (size_t)c.c_hr * c.img_size * c.img_size;
     const size_t n = per_sample * B;
     h->cur_x = h->d_x_work;
     h->cur_eps = h->d_eps;
-    B2D_TRY(run_step_ops(h, st, true));
+    B2D_TRY(run_step_ops(h, st, true, 0, -1, ddim));
     const int blocks = (int)std::min<size_t>((n / 4 + 255) / 256, (size_t)h->num_sms * 8);
-    B2D_TRY(join_temb_side(h, st));   // the update's last block advances d_t, which the side branch reads
-    B2D_CUDA(launch_k(posterior_update_kernel, dim3(blocks), dim3(256), 0, st, h->d_x_work, h->d_eps, h->d_job, h->d_alphas,
-                      h->d_betas, h->d_alpha_hat, h->d_step, h->d_t, B, n, per_sample));
+    B2D_TRY(join_temb_side(h, st));   // the update's last block advances d_t / d_t_next, which the side branch reads
+    if (ddim)
+        B2D_CUDA(launch_k(ddim_update_kernel, dim3(blocks), dim3(256), 0, st, h->d_x_work, h->d_eps, h->d_job, h->d_ddim_tau,
+                          h->d_ddim_coef, h->d_step, h->d_t, h->d_t_next, B, n, per_sample));
+    else
+        B2D_CUDA(launch_k(posterior_update_kernel, dim3(blocks), dim3(256), 0, st, h->d_x_work, h->d_eps, h->d_job, h->d_alphas,
+                          h->d_betas, h->d_alpha_hat, h->d_step, h->d_t, B, n, per_sample));
     return 0;
 }
 
-static int capture_steps(b2d_handle* h, int B, int nsteps, cudaGraphExec_t* out, int* nodes_out) {
+static int capture_steps(b2d_handle* h, int B, int nsteps, bool ddim, cudaGraphExec_t* out, int* nodes_out) {
     cudaStream_t cs = h->own_stream;
     B2D_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
     int rc = 0;
-    for (int s = 0; s < nsteps && rc == 0; ++s) rc = enqueue_reverse_step(h, B, cs);
+    for (int s = 0; s < nsteps && rc == 0; ++s) rc = enqueue_reverse_step(h, B, cs, ddim);
     cudaGraph_t graph = nullptr;
     cudaError_t ce = cudaStreamEndCapture(cs, &graph);
     if (rc) {
@@ -1304,12 +1393,21 @@ static int sample_core(b2d_handle* h, const float* noise, uint64_t seed, uint64_
     job.sample_offset = sample_offset;
     job.noise_stride = per_sample * B;
     job.noise_scale = noise_scale;
-    B2D_CUDA(launch_k(set_job_kernel, dim3(1), dim3(256), 0, st, h->d_job, job, h->d_t, h->d_step, T - 1, B));
+    const bool ddim = h->ddim;
+    int n_evals = T - 1;   // model evaluations of the loop
+    if (ddim) {
+        B2D_TRY(ddim_prepare(h));
+        n_evals = (int)h->ddim_tau.size();
+        B2D_CUDA(launch_k(set_job_ddim_kernel, dim3(1), dim3(256), 0, st, h->d_job, job, h->d_ddim_tau, h->d_t, h->d_t_next,
+                          h->d_step, B));
+    } else {
+        B2D_CUDA(launch_k(set_job_kernel, dim3(1), dim3(256), 0, st, h->d_job, job, h->d_t, h->d_step, T - 1, B));
+    }
     static const bool no_graph = getenv("B2D_NO_GRAPH") != nullptr;   // A/B: plain stream launches (PDL) instead of graphs
     if (temb_pipelined(h)) B2D_TRY(h->step_ops[0](st));   // embeddings of the first step; later ones come from the side branch
     if (no_graph) {
-        for (int i = T - 1; i >= 1; --i) B2D_TRY(enqueue_reverse_step(h, B, st));
-        h->last_launches = ((int64_t)h->step_ops.size() + 1) * (T - 1) + 2;
+        for (int i = 0; i < n_evals; ++i) B2D_TRY(enqueue_reverse_step(h, B, st, ddim));
+        h->last_launches = ((int64_t)h->step_ops.size() + 1) * n_evals + 2;
         return 0;
     }
     static const int env_steps = getenv("B2D_GRAPH_STEPS") ? atoi(getenv("B2D_GRAPH_STEPS")) : 8;
@@ -1318,12 +1416,17 @@ static int sample_core(b2d_handle* h, const float* noise, uint64_t seed, uint64_
         h->drop_graphs();
         h->graph_steps = gs;
     }
-    if (!h->graph_one) B2D_TRY(capture_steps(h, B, 1, &h->graph_one, &h->graph_nodes_one));
-    if (gs > 1 && !h->graph_multi) B2D_TRY(capture_steps(h, B, gs, &h->graph_multi, &h->graph_nodes_multi));
-    const int n_multi = gs > 1 ? (T - 1) / gs : 0, n_one = (T - 1) - n_multi * gs;
-    for (int k = 0; k < n_multi; ++k) B2D_CUDA(cudaGraphLaunch(h->graph_multi, st));
-    for (int k = 0; k < n_one; ++k) B2D_CUDA(cudaGraphLaunch(h->graph_one, st));
-    h->last_launches = (int64_t)h->graph_nodes_multi * n_multi + (int64_t)h->graph_nodes_one * n_one + 2;
+    // each mode replays its own pair; capturing one pair leaves the other untouched
+    cudaGraphExec_t& g_one = ddim ? h->graph_one_ddim : h->graph_one;
+    cudaGraphExec_t& g_multi = ddim ? h->graph_multi_ddim : h->graph_multi;
+    int& nodes_one = ddim ? h->graph_nodes_one_ddim : h->graph_nodes_one;
+    int& nodes_multi = ddim ? h->graph_nodes_multi_ddim : h->graph_nodes_multi;
+    if (!g_one) B2D_TRY(capture_steps(h, B, 1, ddim, &g_one, &nodes_one));
+    if (gs > 1 && !g_multi) B2D_TRY(capture_steps(h, B, gs, ddim, &g_multi, &nodes_multi));
+    const int n_multi = gs > 1 ? n_evals / gs : 0, n_one = n_evals - n_multi * gs;
+    for (int k = 0; k < n_multi; ++k) B2D_CUDA(cudaGraphLaunch(g_multi, st));
+    for (int k = 0; k < n_one; ++k) B2D_CUDA(cudaGraphLaunch(g_one, st));
+    h->last_launches = (int64_t)nodes_multi * n_multi + (int64_t)nodes_one * n_one + 2;
     return 0;
 }
 
@@ -1362,7 +1465,8 @@ static int sample_host_enqueue(b2d_handle* h, float* x_inout_host, const float* 
     if (topo_host) B2D_CUDA(cudaMemcpyAsync(h->d_topo_stage, topo_host, (size_t)B * plane * 4, cudaMemcpyHostToDevice, st));
     if (cond_host) B2D_CUDA(cudaMemcpyAsync(h->d_cond_stage, cond_host, cond_elems * 4, cudaMemcpyHostToDevice, st));
     if (noise_host) {
-        const size_t ne = (size_t)h->T * n;
+        // [T][n] indexed by i for the DDPM loop, [S][n] indexed by k for the DDIM loop (S <= T-1 fits the same staging)
+        const size_t ne = (h->ddim ? h->ddim_tau.size() : (size_t)h->T) * n;
         if (ne > h->noise_stage_elems) {
             B2D_CUDA(cudaStreamSynchronize(st));
             h->release(h->d_noise_stage);
@@ -1672,6 +1776,47 @@ int b2d_op_posterior_update(float* x, const float* eps, const float* z, const fl
     const int blocks = (int)std::min<size_t>((n / 4 + 255) / 256, (size_t)148 * 8);
     B2D_CUDA(launch_k(posterior_update_kernel, dim3(blocks), dim3(256), 0, st, x, eps, sc.job, alphas, betas, alpha_hat, sc.step, nullptr, B, n,
                       (size_t)per_sample));
+    B2D_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int b2d_op_ddim_update(float* x, const float* eps, const float* z_or_null, const float* alpha_hat, int32_t T, int32_t t,
+                       int32_t t_prev, float eta, int32_t B, int64_t per_sample, uint64_t seed, uint64_t sample_offset,
+                       float noise_scale, void* stream) {
+    B2D_CHECK(x && eps && alpha_hat && B >= 1 && per_sample >= 1 && T >= 2, "bad argument");
+    B2D_CHECK(per_sample % 4 == 0, "per-sample element count must be a multiple of 4 (vectorised update)");
+    B2D_CHECK(t >= 1 && t <= T - 1, "t must lie in [1, T-1]");
+    B2D_CHECK(t_prev == -1 || (t_prev >= 1 && t_prev < t), "t_prev must be -1 (final step) or lie in [1, t-1]");
+    B2D_CHECK(eta >= 0.f && eta <= 1.f, "eta must lie in [0, 1]");
+    cudaStream_t st = as_stream(stream);
+    // the coefficients come from the fp32 alpha_hat values the caller's table holds, through the same host function as the
+    // handle's per-step table
+    float ah[2] = {0.f, 1.f};
+    B2D_CUDA(cudaMemcpyAsync(&ah[0], alpha_hat + t, 4, cudaMemcpyDeviceToHost, st));
+    if (t_prev >= 1) B2D_CUDA(cudaMemcpyAsync(&ah[1], alpha_hat + t_prev, 4, cudaMemcpyDeviceToHost, st));
+    B2D_CUDA(cudaStreamSynchronize(st));
+    const float4 c = ddim_coefficients(ah[0], ah[1], eta);
+    // persistent scratch of this entry point (step index, job block, one-row tables), written in stream order
+    struct Scratch { int* step = nullptr; SampleJob* job = nullptr; int* tau = nullptr; float4* coef = nullptr; };
+    static thread_local Scratch sc;
+    if (!sc.step) {
+        B2D_CUDA(cudaMalloc(&sc.step, 16));
+        B2D_CUDA(cudaMalloc(&sc.job, sizeof(SampleJob)));
+        B2D_CUDA(cudaMalloc(&sc.tau, 16));
+        B2D_CUDA(cudaMalloc(&sc.coef, sizeof(float4)));
+    }
+    const size_t n = (size_t)B * per_sample;
+    SampleJob job{};
+    job.noise = z_or_null;   // the noise of THIS step: k = 0
+    job.seed = seed;
+    job.sample_offset = sample_offset;
+    job.noise_stride = n;
+    job.noise_scale = noise_scale;
+    ddim_op_setup_kernel<<<1, 32, 0, st>>>(sc.job, job, sc.step, sc.tau, sc.coef, (int)t, c);
+    B2D_CUDA(cudaGetLastError());
+    const int blocks = (int)std::min<size_t>((n / 4 + 255) / 256, (size_t)148 * 8);
+    B2D_CUDA(launch_k(ddim_update_kernel, dim3(blocks), dim3(256), 0, st, x, eps, sc.job, sc.tau, sc.coef, sc.step, nullptr, nullptr, B,
+                      n, (size_t)per_sample));
     B2D_CUDA(cudaGetLastError());
     return 0;
 }

@@ -1,6 +1,9 @@
 // HBM/latency-bound kernels of the sampling step: time embeddings + projections, the 8x8/s2 stem convolution on the
-// fp32 state, InstanceNorm statistics/apply, the Cout=1 tail convolution and the DDPM posterior update.
+// fp32 state, InstanceNorm statistics/apply, the Cout=1 tail convolution, the DDPM posterior update and the DDIM update.
 #pragma once
+#include <algorithm>
+#include <cmath>
+
 #include "common.cuh"
 
 namespace b2d {
@@ -783,6 +786,120 @@ __global__ void __launch_bounds__(256) posterior_update_kernel(float* __restrict
         }
     }
 }
+
+// ------------------------------------------------------------------------------------------------ DDIM update
+// Song, Meng & Ermon 2021, eq. 12, over a strided timestep sequence tau_0 > tau_1 > ... > tau_{S-1} (every tau_k in [1, T-1]).
+// Step k goes from t = tau_k to t' = tau_{k+1}; a = alpha_hat[t], a' = alpha_hat[t'] (a' = 1 after the last step: x0_hat):
+//   x0_hat = (x - sqrt(1-a) eps) / sqrt(a)
+//   sigma  = eta * sqrt((1-a')/(1-a)) * sqrt(1 - a/a')
+//   x'     = sqrt(a') x0_hat + sqrt(max(0, 1-a'-sigma^2)) eps + sigma * noise_scale * z
+// folded into x' = cx x + ce eps + sigma (noise_scale z) with cx = sqrt(a'/a) and ce = sqrt(max(0, 1-a'-sigma^2)) - cx sqrt(1-a).
+// The coefficients are computed here, on the host, in double from the fp32 alpha_hat values: the square roots of differences of
+// nearby alpha_hat values lose most of their bits in fp32.  Both the handle's per-step table and b2d_op_ddim_update use this
+// function.  No x0_hat clipping (the reference has none); sigma is 0 on the last step and for eta = 0, so no noise is drawn there.
+inline float4 ddim_coefficients(float abar, float abar_next, float eta) {
+    const double a = abar, an = abar_next;
+    const double sigma = (double)eta * std::sqrt((1.0 - an) / (1.0 - a)) * std::sqrt(std::max(0.0, 1.0 - a / an));
+    const double cx = std::sqrt(an / a);
+    const double ce = std::sqrt(std::max(0.0, 1.0 - an - sigma * sigma)) - cx * std::sqrt(1.0 - a);
+    return make_float4((float)cx, (float)ce, (float)sigma, 0.f);
+}
+
+// Reverse-loop state of a DDIM job: k = 0, t[b] = tau_0 for the first evaluation, t_next[b] = tau_1 for the time-embedding
+// side branch that runs before the first update.  tau is the device table [S + 2] (two trailing zeros).
+__global__ void set_job_ddim_kernel(SampleJob* job, SampleJob v, const int* __restrict__ tau, int* t_arr, int* t_next_arr,
+                                    int* step_ptr, int B) {
+    pdl_launch_dependents();
+    pdl_wait();
+    if (threadIdx.x == 0) {
+        *job = v;
+        step_ptr[0] = 0;
+        step_ptr[1] = 0;
+    }
+    const int t0 = tau[0], t1 = tau[1];
+    for (int b = threadIdx.x; b < B; b += blockDim.x) {
+        t_arr[b] = t0;
+        t_next_arr[b] = t1;
+    }
+}
+
+// State, sequence and coefficients of one stand-alone step (b2d_op_ddim_update), written in stream order.
+__global__ void ddim_op_setup_kernel(SampleJob* job, SampleJob v, int* step_ptr, int* tau, float4* coef, int t, float4 c) {
+    if (threadIdx.x == 0) {
+        *job = v;
+        step_ptr[0] = 0;
+        step_ptr[1] = 0;
+        tau[0] = t;
+        coef[0] = c;
+    }
+}
+
+// step_ptr[0] holds k; tau [S + 2] and coef [S] = {cx, ce, sigma, 0} are device tables written by the host.  z is host-injected
+// (noise[k][...]) or drawn from the same Philox stream as posterior_update_kernel with the step slot set to tau_k.  Inside the
+// reverse loop (t_arr != nullptr) the last block to arrive writes t[b] = tau_{k+1} (the next evaluation) and
+// t_next[b] = tau_{k+2} (the time embeddings the side branch of that evaluation precomputes), then k <- k+1.
+__global__ void __launch_bounds__(256) ddim_update_kernel(float* __restrict__ x, const float* __restrict__ eps,
+                                                          const SampleJob* __restrict__ job, const int* __restrict__ tau,
+                                                          const float4* __restrict__ coef, int* __restrict__ step_ptr,
+                                                          int* __restrict__ t_arr, int* __restrict__ t_next_arr, int B, size_t n,
+                                                          size_t per_sample) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int k = *step_ptr;
+    const int t = tau[k];
+    const float4 c = coef[k];
+    const float* noise = job->noise;
+    const unsigned long long seed = job->seed, sample_offset = job->sample_offset;
+    const size_t noise_stride = job->noise_stride;
+    const float noise_scale = job->noise_scale;
+    const bool draw = c.z != 0.f;
+    const size_t n4 = n >> 2;
+    for (size_t v = blockIdx.x * (size_t)blockDim.x + threadIdx.x; v < n4; v += (size_t)gridDim.x * blockDim.x) {
+        float4 xv = reinterpret_cast<float4*>(x)[v];
+        const float4 ev = reinterpret_cast<const float4*>(eps)[v];
+        float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (draw) {
+            if (noise) {
+                zv = reinterpret_cast<const float4*>(noise + (size_t)k * noise_stride)[v];
+                zv = make_float4(zv.x * noise_scale, zv.y * noise_scale, zv.z * noise_scale, zv.w * noise_scale);
+            } else {
+                const size_t e = v * 4;
+                const unsigned long long sample = sample_offset + e / per_sample;
+                const unsigned long long within = (e % per_sample) >> 2;
+                uint32_t ctr[4] = {(uint32_t)within, (uint32_t)t, (uint32_t)sample, (uint32_t)(sample >> 32)};
+                philox4x32_10(ctr, (uint32_t)seed, (uint32_t)(seed >> 32));
+                const float2 g0 = box_muller(ctr[0], ctr[1]), g1 = box_muller(ctr[2], ctr[3]);
+                zv = make_float4(g0.x * noise_scale, g0.y * noise_scale, g1.x * noise_scale, g1.y * noise_scale);
+            }
+        }
+        xv.x = fmaf(c.z, zv.x, fmaf(c.y, ev.x, c.x * xv.x));
+        xv.y = fmaf(c.z, zv.y, fmaf(c.y, ev.y, c.x * xv.y));
+        xv.z = fmaf(c.z, zv.z, fmaf(c.y, ev.z, c.x * xv.z));
+        xv.w = fmaf(c.z, zv.w, fmaf(c.y, ev.w, c.x * xv.w));
+        reinterpret_cast<float4*>(x)[v] = xv;
+    }
+    if (t_arr != nullptr) {
+        __shared__ bool s_last;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            __threadfence();
+            s_last = atomicAdd(reinterpret_cast<unsigned int*>(step_ptr + 1), 1u) == gridDim.x - 1;
+        }
+        __syncthreads();
+        if (s_last) {
+            const int t1 = tau[k + 1], t2 = tau[k + 2];
+            for (int b = threadIdx.x; b < B; b += blockDim.x) {
+                t_arr[b] = t1;
+                t_next_arr[b] = t2;
+            }
+            if (threadIdx.x == 0) {
+                step_ptr[0] = k + 1;
+                step_ptr[1] = 0;
+            }
+        }
+    }
+}
+
 // x_T ~ N(0,1) * scale drawn on the device (ensemble driver): same Philox keying as the per-step noise — (seed; global sample
 // index, element) — with the step slot set to 0x7FFFFFFF, which no reverse step uses, so members are independent of how the
 // ensemble is cut into sub-batches and ranks.

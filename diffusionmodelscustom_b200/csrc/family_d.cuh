@@ -545,7 +545,7 @@ static int build_program_d(Handle* h, int B) {
         ops.meta("temb", "temb_project", 2.0 * B * TS * 256, 4.0 * TS * 256);
         ops.push_back([=](cudaStream_t st) {
             dim3 grid((TS + TEMB_OC - 1) / TEMB_OC, (B + TEMB_SB - 1) / TEMB_SB);
-            B2D_CUDA(launch_k(temb_project_kernel, grid, dim3(256), 0, st, hh->d_t, nullptr, nullptr, ei, dd, tw, tb, temb, TS, TS, B, hh->temb_t_off, 0));
+            B2D_CUDA(launch_k(temb_project_kernel, grid, dim3(256), 0, st, hh->temb_t, nullptr, nullptr, ei, dd, tw, tb, temb, TS, TS, B, hh->temb_t_off, 0));
             return 0;
         });
     }

@@ -8,10 +8,13 @@ cond_img, lsm_cond, topo_cond)``); ``DiffusionUtilsV2`` mirrors DDPM_clean_appli
 The schedule tables are built with the same torch expressions as the reference (they are part of the public attribute
 surface: ``.betas/.alphas/.alpha_hat``).  The reverse loop itself runs natively: one captured CUDA graph per step, replayed
 T-1 times, with the posterior update and (optionally) the Philox normal draws in ``posterior_update_kernel``.
+``DiffusionUtils.sample_ddim`` (not in the reference) runs the DDIM sampler over S << T timesteps of the same schedule through the
+same graphs, with ``ddim_update_kernel`` in place of the posterior update.
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -19,6 +22,18 @@ import torch.nn as nn
 
 from . import _native as N
 from .modules import NativeModel
+
+
+def ddim_coefficients(alpha_hat, t: int, t_prev: int, eta: float):
+    """(cx, ce, sigma) of one DDIM step, x' = cx x + ce eps_hat + sigma z: a Python mirror, in double from the fp32 table, of
+    ``ddim_coefficients()`` in csrc/elementwise.cuh (the function the native per-step table and ``b2d_op_ddim_update`` use).
+    ``t_prev = -1`` is the final step (alpha_hat' = 1)."""
+    a = float(np.float32(alpha_hat[t]))
+    an = 1.0 if t_prev < 0 else float(np.float32(alpha_hat[t_prev]))
+    sigma = float(np.float32(eta)) * math.sqrt((1.0 - an) / (1.0 - a)) * math.sqrt(max(0.0, 1.0 - a / an))
+    cx = math.sqrt(an / a)
+    ce = math.sqrt(max(0.0, 1.0 - an - sigma * sigma)) - cx * math.sqrt(1.0 - a)
+    return float(np.float32(cx)), float(np.float32(ce)), float(np.float32(sigma))
 
 
 class DiffusionUtils:
@@ -78,7 +93,7 @@ class DiffusionUtils:
         return (alpha_hat_sqrts * x) + (one_minus_alpha_hat_sqrt * noise), noise
 
     # ------------------------------------------------------------------ reverse process
-    def _run(self, x, model, y, cond_img, lsm_cond, topo_cond, noise, seed, sample_offset):
+    def _run(self, x, model, y, cond_img, lsm_cond, topo_cond, noise, seed, sample_offset, ddim=None):
         assert len(x.shape) == 4, 'x must be a 4D tensor'
         if not x.is_cuda:
             raise N.NativeError("sampling runs only on CUDA (sm_100a); there is no CPU path")
@@ -90,7 +105,9 @@ class DiffusionUtils:
         model.eval()
         if isinstance(model, NativeModel):
             out = model.native_sample(x, y, cond_img, lsm_cond, topo_cond, self.betas, self.alphas, self.alpha_hat,
-                                      noise=noise, seed=seed, sample_offset=sample_offset, noise_scale=scale)
+                                      noise=noise, seed=seed, sample_offset=sample_offset, noise_scale=scale, ddim=ddim)
+        elif ddim is not None:
+            out = self._foreign_ddim_loop(x, model, y, cond_img, lsm_cond, topo_cond, noise, seed, sample_offset, scale, ddim)
         else:
             out = self._foreign_model_loop(x, model, y, cond_img, lsm_cond, topo_cond, noise, seed, sample_offset, scale)
         return out, was_training
@@ -112,6 +129,67 @@ class DiffusionUtils:
                                                   int(sample_offset), float(scale),
                                                   torch.cuda.current_stream().cuda_stream))
         return x
+
+    def _foreign_ddim_loop(self, x, model, y, cond_img, lsm_cond, topo_cond, noise, seed, sample_offset, scale, ddim):
+        """Any other callable eps-model under DDIM: python loop over the model, native DDIM-update kernel."""
+        L = N.lib()
+        dev = x.device
+        ts, eta = ddim
+        ahat = self.alpha_hat.detach().to(dev, torch.float32).contiguous()
+        B = x.shape[0]
+        per = x[0].numel()
+        with torch.no_grad(), torch.cuda.device(dev):
+            for k, t in enumerate(ts):
+                t_prev = ts[k + 1] if k + 1 < len(ts) else -1
+                tt = torch.full((B,), t, dtype=torch.long, device=dev)
+                eps = model(x, tt, y, cond_img, lsm_cond, topo_cond).to(torch.float32).contiguous()
+                z = None if noise is None else noise[k].to(dev, torch.float32).contiguous()
+                N.check(L.b2d_op_ddim_update(x.data_ptr(), eps.data_ptr(), N.ptr(z), ahat.data_ptr(), self.n_timesteps, t,
+                                             t_prev, float(eta), B, per, int(seed), int(sample_offset), float(scale),
+                                             torch.cuda.current_stream().cuda_stream))
+        return x
+
+    def ddim_timesteps(self, steps: int):
+        """Default DDIM sequence for ``steps`` = S evaluations: tau_k = (T-1) - floor(k (T-2) / (S-1)), k = 0 ... S-1, so
+        tau_0 = T-1 and tau_{S-1} = 1 ([T-1] for S = 1).  Integer arithmetic: strictly decreasing for every 2 <= S <= T-1."""
+        T = self.n_timesteps
+        steps = int(steps)
+        if not 1 <= steps <= T - 1:
+            raise ValueError(f"steps must lie in [1, {T - 1}] (T = {T}), got {steps}")
+        if steps == 1:
+            return [T - 1]
+        return [(T - 1) - (k * (T - 2)) // (steps - 1) for k in range(steps)]
+
+    def _ddim_plan(self, steps, eta, timesteps):
+        """(sequence, eta) of a DDIM run: ``timesteps`` if given (validated), else the default sequence for ``steps``."""
+        eta = float(eta)
+        if not 0.0 <= eta <= 1.0:
+            raise ValueError(f"eta must lie in [0, 1], got {eta}")
+        if timesteps is None:
+            return self.ddim_timesteps(steps), eta
+        ts = [int(t) for t in (timesteps.tolist() if isinstance(timesteps, torch.Tensor) else timesteps)]
+        T = self.n_timesteps
+        if not ts:
+            raise ValueError("timesteps is empty")
+        if any(not 1 <= t <= T - 1 for t in ts):
+            raise ValueError(f"timesteps must lie in [1, {T - 1}] (T = {T})")
+        if any(b >= a for a, b in zip(ts, ts[1:])):
+            raise ValueError("timesteps must be strictly decreasing")
+        return ts, eta
+
+    def sample_ddim(self, x: torch.Tensor, model: nn.Module, y: torch.Tensor = None, cond_img: torch.Tensor = None,
+                    lsm_cond: torch.Tensor = None, topo_cond: torch.Tensor = None, *, steps: int = 50, eta: float = 0.0,
+                    timesteps=None, noise: torch.Tensor = None, seed: int = None, sample_offset: int = 0):
+        """DDIM (Song, Meng & Ermon 2021, eq. 12) with this object's trained-DDPM schedule: x is x_T, returns x_0 after S model
+        evaluations instead of T-1.  Not in the reference.
+
+        ``timesteps`` is a strictly decreasing sequence in [1, T-1]; without it the default ``ddim_timesteps(steps)`` is used.
+        ``eta`` = 0 is the deterministic sampler, 1 has the DDPM posterior variance for consecutive steps.  ``noise``
+        [S,B,C,H,W] injects z indexed by step k; otherwise z is drawn in-kernel from the same Philox stream as ``sample``,
+        with the step slot set to the timestep.  The data_scaled factor multiplies z as in ``sample``; no x_0 clipping."""
+        out, _ = self._run(x, model, y, cond_img, lsm_cond, topo_cond, noise, seed, sample_offset,
+                           ddim=self._ddim_plan(steps, eta, timesteps))
+        return out
 
     def sample(self, x: torch.Tensor, model: nn.Module, y: torch.Tensor = None, cond_img: torch.Tensor = None,
                lsm_cond: torch.Tensor = None, topo_cond: torch.Tensor = None, *, noise: torch.Tensor = None,

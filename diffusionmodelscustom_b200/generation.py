@@ -62,13 +62,17 @@ def _host_f32(t, name, shape_tail=None):
 @torch.no_grad()
 def generate_ensemble(model: NativeModel, diffusion, n_dates: int, members: int, *, season=None, cond_img=None, lsm=None,
                       topo=None, channels_hr: int = 1, img_size: Optional[int] = None, sub_batch: int = 64, seed: int = 0,
-                      device="cuda", group=None, gather: bool = True, return_stats: bool = False):
+                      device="cuda", group=None, gather: bool = True, return_stats: bool = False, steps: Optional[int] = None,
+                      eta: float = 0.0, timesteps=None):
     """Sample ``members`` fields for each of ``n_dates`` conditioning sets.
 
     ``season`` [D] int64, ``cond_img`` [D,C,H,W] (Family D: the low-resolution field [D,C,h,w]), ``lsm`` / ``topo`` [D,1,H,W]:
     HOST tensors, one row per date.  Returns a host tensor [n_dates, members, channels_hr, H, W] (rank-local slice only when
     ``gather=False``).  Under ``torch.distributed`` the flattened member list is cut into contiguous per-rank blocks
-    (``sharding.shard_range``) with no data-path collective; one ``all_gather`` of the final fields."""
+    (``sharding.shard_range``) with no data-path collective; one ``all_gather`` of the final fields.
+
+    ``steps`` / ``timesteps`` (with ``eta``) sample every member with ``diffusion.sample_ddim``'s DDIM loop instead of the DDPM
+    loop of ``diffusion.sample``; ``None`` for both keeps the DDPM loop."""
     if not isinstance(model, NativeModel):
         raise TypeError("generate_ensemble needs a native model (DiffusionNet / UNet_downscale of this package)")
     device = torch.device(device)
@@ -81,6 +85,7 @@ def generate_ensemble(model: NativeModel, diffusion, n_dates: int, members: int,
     total = n_dates * members
     lo, hi = shard_range(total, world, rank)
     sub_batch = max(1, min(sub_batch, max(hi - lo, 1)))
+    ddim = None if (steps is None and timesteps is None) else diffusion._ddim_plan(steps, eta, timesteps)
     model.eval()
     if hasattr(model, "_bind"):            # Family D binds its high-resolution channel count from x
         model._bind(torch.empty(1, channels_hr, H, H))
@@ -104,6 +109,7 @@ def generate_ensemble(model: NativeModel, diffusion, n_dates: int, members: int,
     L.b2d_ensemble_run.argtypes = [C.c_void_p, C.POINTER(EnsembleJob), C.POINTER(EnsembleStats)]
     with torch.cuda.device(device):
         model._set_schedule(h, diffusion.betas, diffusion.alphas, diffusion.alpha_hat)
+        model._set_sampler(h, ddim)
         model._cond_key = None       # the handle's conditioning is overwritten by the driver
         N.check(L.b2d_ensemble_run(h, C.byref(job), C.byref(stats)))
     if gather and world > 1:

@@ -301,6 +301,16 @@ class NativeModel(nn.Module):
             N.check(N.lib().b2d_set_schedule(h, b.data_ptr(), a.data_ptr(), ah.data_ptr(), len(b)))
             self._sched_key = skey
 
+    def _set_sampler(self, h, ddim=None):
+        """Sampler mode of the handle for the next native loop: ``None`` = the reference DDPM loop, ``(timesteps, eta)`` = DDIM
+        over that sequence (b2d_set_timesteps).  Every native sampling call sets it, so no mode leaks from one call to the next."""
+        if ddim is None:
+            N.check(N.lib().b2d_set_timesteps(h, None, 0, 0.0))
+            return
+        ts, eta = ddim
+        arr = (C.c_int32 * len(ts))(*[int(t) for t in ts])
+        N.check(N.lib().b2d_set_timesteps(h, arr, len(ts), float(eta)))
+
     def launch_count(self) -> int:
         return 0 if self._h is None else int(N.lib().b2d_last_launch_count(self._h))
 
@@ -371,7 +381,7 @@ class DiffusionNet(NativeModel):
 
     @torch.no_grad()
     def native_sample(self, x, y, cond_img, lsm_cond, topo_cond, betas, alphas, alpha_hat, noise=None, seed=0,
-                      sample_offset=0, noise_scale=1.0):
+                      sample_offset=0, noise_scale=1.0, ddim=None):
         """Whole reverse loop on the device (CUDA graph); x is updated in place and returned."""
         B, _, H, _ = x.shape
         h = self._ensure(B, H, x.device)
@@ -380,6 +390,7 @@ class DiffusionNet(NativeModel):
         with torch.cuda.device(x.device):
             stream = torch.cuda.current_stream().cuda_stream
             self._set_schedule(h, betas, alphas, alpha_hat)
+            self._set_sampler(h, ddim)
             self._set_conditioning(h, B, y, cond_img, lsm_cond, topo_cond, stream)
             nz = self._f32c(noise, "noise")
             N.check(N.lib().b2d_sample(h, x.data_ptr(), N.ptr(nz), int(seed), int(sample_offset), float(noise_scale), B,
@@ -390,7 +401,7 @@ class DiffusionNet(NativeModel):
 
     @torch.no_grad()
     def native_sample_host(self, x_host, y, cond_img, lsm_cond, topo_cond, betas, alphas, alpha_hat, device, noise=None,
-                           seed=0, sample_offset=0, noise_scale=1.0):
+                           seed=0, sample_offset=0, noise_scale=1.0, ddim=None):
         """End-to-end entry on HOST tensors (b2d_sample_host): H2D of x_T/conditioning, the whole loop, D2H of x_0."""
         B, _, H, _ = x_host.shape
         device = torch.device(device)
@@ -409,6 +420,7 @@ class DiffusionNet(NativeModel):
         cond, yy, nz = hostc(cond_img), hostc(y, torch.int64), hostc(noise)
         with torch.cuda.device(device):
             self._set_schedule(h, betas, alphas, alpha_hat)
+            self._set_sampler(h, ddim)
             self._cond_key = None   # conditioning of the handle is overwritten by this call
             N.check(N.lib().b2d_sample_host(h, out.data_ptr(), N.ptr(lsm), N.ptr(topo), N.ptr(cond), 0, 0, N.ptr(yy),
                                             N.ptr(nz), int(seed), int(sample_offset), float(noise_scale), B))

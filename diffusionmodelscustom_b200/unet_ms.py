@@ -130,7 +130,7 @@ class UNet_downscale(NativeModel):
 
     @torch.no_grad()
     def native_sample(self, x, y, cond_img, lsm_cond, topo_cond, betas, alphas, alpha_hat, noise=None, seed=0,
-                      sample_offset=0, noise_scale=1.0):
+                      sample_offset=0, noise_scale=1.0, ddim=None):
         self._bind(x)
         B, _, H, _ = x.shape
         h = self._ensure(B, H, x.device)
@@ -139,6 +139,7 @@ class UNet_downscale(NativeModel):
         with torch.cuda.device(x.device):
             stream = torch.cuda.current_stream().cuda_stream
             self._set_schedule(h, betas, alphas, alpha_hat)
+            self._set_sampler(h, ddim)
             self._set_conditioning(h, B, y, cond_img, None, None, stream)
             nz = self._f32c(noise, "noise")
             N.check(N.lib().b2d_sample(h, x.data_ptr(), N.ptr(nz), int(seed), int(sample_offset), float(noise_scale), B,
@@ -149,7 +150,7 @@ class UNet_downscale(NativeModel):
 
     @torch.no_grad()
     def native_sample_host(self, x_host, y, cond_img, lsm_cond, topo_cond, betas, alphas, alpha_hat, device, noise=None,
-                           seed=0, sample_offset=0, noise_scale=1.0):
+                           seed=0, sample_offset=0, noise_scale=1.0, ddim=None):
         self._bind(x_host)
         B, _, H, _ = x_host.shape
         device = torch.device(device)
@@ -160,6 +161,7 @@ class UNet_downscale(NativeModel):
         ch, cw = (0, 0) if lowc is None else (lowc.shape[-2], lowc.shape[-1])
         with torch.cuda.device(device):
             self._set_schedule(h, betas, alphas, alpha_hat)
+            self._set_sampler(h, ddim)
             self._cond_key = None
             N.check(N.lib().b2d_sample_host(h, out.data_ptr(), None, None, N.ptr(lowc), ch, cw, None, N.ptr(nz), int(seed),
                                             int(sample_offset), float(noise_scale), B))

@@ -102,6 +102,26 @@ int b2d_decoder_forward(b2d_handle* h, const float* const* fmaps_in, const int64
 int b2d_sample(b2d_handle* h, float* x_inout, const float* noise, uint64_t seed, uint64_t sample_offset,
                float noise_scale, int32_t B, void* stream);
 
+/* ---- fewer-step sampling: DDIM (Song, Meng & Ermon 2021, eq. 12) ------------------------------------------------------
+ * Over a strictly decreasing timestep sequence tau_0 > ... > tau_{S-1} (each in [1, T-1]) and eta in [0, 1], step k goes from
+ * t = tau_k to t' = tau_{k+1} with a = alpha_hat[t], a' = alpha_hat[t'] (a' = 1 after the last step, whose result is x0_hat):
+ *   x0_hat = (x - sqrt(1-a) eps_hat) / sqrt(a)
+ *   sigma  = eta * sqrt((1-a')/(1-a)) * sqrt(1 - a/a')
+ *   x'     = sqrt(a') x0_hat + sqrt(max(0, 1-a'-sigma^2)) eps_hat + sigma * noise_scale * z
+ * No x0_hat clipping; the last step draws no noise.  z is Philox keyed by (seed; sample_offset + sample, element) with the step
+ * slot set to tau_k, or injected noise [S][B*c_hr*H*W] indexed by k.
+ * b2d_set_timesteps switches the handle's sampler: b2d_sample, b2d_sample_host and b2d_ensemble_run then run S evaluations of
+ * the DDIM loop instead of the T-1 of the DDPM loop.  The two loops keep separate step graphs. */
+/* n == 0 (timesteps NULL) restores the reference DDPM loop.  Validated: strictly decreasing, 1 <= t <= T-1, 0 <= eta <= 1;
+ * re-validated at sampling time against the current schedule length. */
+int b2d_set_timesteps(b2d_handle* h, const int32_t* timesteps_host, int32_t n, float eta);
+/* One DDIM step on device memory (foreign-model loop, op tests).  t_prev = -1: final step to x0 (alpha_hat' = 1).
+ * alpha_hat: device fp32 [T]; z_or_null: this step's z [B*per_sample] or NULL for Philox.  Synchronises `stream` once (reads
+ * alpha_hat[t] and alpha_hat[t_prev] back for the coefficients). */
+int b2d_op_ddim_update(float* x, const float* eps, const float* z_or_null, const float* alpha_hat, int32_t T, int32_t t,
+                       int32_t t_prev, float eta, int32_t B, int64_t per_sample, uint64_t seed, uint64_t sample_offset,
+                       float noise_scale, void* stream);
+
 /* End-to-end entry with HOST buffers: uploads x_T and the conditioning, runs b2d_sample, downloads x_0, synchronises. */
 int b2d_sample_host(b2d_handle* h, float* x_inout_host, const float* lsm_host, const float* topo_host,
                     const float* cond_host, int32_t cond_h, int32_t cond_w, const int64_t* y_host,
