@@ -604,20 +604,31 @@ static int build_program_d(Handle* h, int B) {
         bd.attention(in, hw, C, role, o, 0);
         return o;
     };
-    f16* x2 = sa(down(x1, H, 64, 128, "down1", D_TEMB_OFF[0]), H / 2, 128, "sa1");
-    f16* x3 = sa(down(x2, H / 2, 128, 256, "down2", D_TEMB_OFF[1]), H / 4, 256, "sa2");
-    f16* x4 = sa(down(x3, H / 4, 256, 256, "down3", D_TEMB_OFF[2]), H / 8, 256, "sa3");
+    f16* x2_pre = down(x1, H, 64, 128, "down1", D_TEMB_OFF[0]);
+    f16* x2 = sa(x2_pre, H / 2, 128, "sa1");
+    f16* x3_pre = down(x2, H / 2, 128, 256, "down2", D_TEMB_OFF[1]);
+    f16* x3 = sa(x3_pre, H / 4, 256, "sa2");
+    f16* x4_pre = down(x3, H / 4, 256, 256, "down3", D_TEMB_OFF[2]);
+    f16* x4 = sa(x4_pre, H / 8, 256, "sa3");
+    h->taps["x2_pre"] = {x2_pre, 128, H / 2};
+    h->taps["x3_pre"] = {x3_pre, 256, H / 4};
+    h->taps["x4_pre"] = {x4_pre, 256, H / 8};
     h->taps["x2"] = {x2, 128, H / 2};
     h->taps["x3"] = {x3, 256, H / 4};
     h->taps["x4"] = {x4, 256, H / 8};
     x4 = bd.double_conv(x4, H / 8, 256, 256, 256, "bot1", false, nullptr, 0);
     x4 = bd.double_conv(x4, H / 8, 256, 256, 256, "bot3", false, nullptr, 0);
     h->taps["bot"] = {x4, 256, H / 8};
-    f16* u1 = sa(up(x4, H / 8, 256, x3, 256, 128, "up1", D_TEMB_OFF[3]), H / 4, 128, "sa4");
-    f16* u2 = sa(up(u1, H / 4, 128, x2, 128, 64, "up2", D_TEMB_OFF[4]), H / 2, 64, "sa5");
+    f16* u1_pre = up(x4, H / 8, 256, x3, 256, 128, "up1", D_TEMB_OFF[3]);
+    f16* u1 = sa(u1_pre, H / 4, 128, "sa4");
+    f16* u2_pre = up(u1, H / 4, 128, x2, 128, 64, "up2", D_TEMB_OFF[4]);
+    f16* u2 = sa(u2_pre, H / 2, 64, "sa5");
     f16* u3_pre = up(u2, H / 2, 64, x1, 64, 64, "up3", D_TEMB_OFF[5]);
     h->temb_free_op = (int)ops.v.size();   // nothing below reads d_temb
     f16* u3 = sa(u3_pre, H, 64, "sa6");
+    h->taps["u1_pre"] = {u1_pre, 128, H / 4};
+    h->taps["u2_pre"] = {u2_pre, 64, H / 2};
+    h->taps["u3_pre"] = {u3_pre, 64, H};
     h->taps["u1"] = {u1, 128, H / 4};
     h->taps["u2"] = {u2, 64, H / 2};
     h->taps["u3"] = {u3, 64, H};
